@@ -8,8 +8,10 @@ stage-3 weights of configs/fit_rgb_demo_use_split.cfg), synthetic seeded inputs 
 
     python bench.py --gpus N --steps K --warmup W            # this repo's arm
     python bench.py --impl reference ...                     # the reference algorithm on the host CPUs (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write what the last timed step returned, as DIR/*.npy
 """
 import argparse
+import hashlib
 import json
 import os
 import subprocess
@@ -28,6 +30,8 @@ from humor_b200 import synth  # noqa: E402
 LBS_BYTES_FWD = 83896          # SURVEY.md §8(d): per frame, fwd (inputs + v + Jtr)
 LBS_BYTES_BWD = 84236
 METRIC = 'stage3_optimizer_step_frames_per_sec'
+DUMP_LIMIT_BYTES = 64_000_000
+NPY_HEADER_BYTES = 128          # np.save's header for arrays of up to four dimensions
 
 
 def load_peaks():
@@ -120,26 +124,40 @@ def make_optimizer(B, T, prob, dev, config='rgb'):
 OBS_KEYS = ('joints2d', 'floor_plane', 'seq_interval')
 
 
-def project_obs_from_product(mo, prob, dev, config='rgb'):
-    """Informative observations: the product's own prediction at the initial state + noise (2-D keypoints for the RGB config,
-    key vertices with the synthetic occlusion mask for the AMASS config)."""
-    keys = CONFIGS[config]['obs']
-    mo.set_stage3_state(prob['params'])
-    obs = {k: torch.as_tensor(prob['obs'][k]).to(dev) for k in keys}
+def project_obs(prob, config='rgb'):
+    """Informative observations: the prediction at the seeded initial state + seeded noise (2-D keypoints for the RGB config,
+    key vertices with the synthetic occlusion mask for the AMASS config).  The prediction is the oracle port's forward (plain
+    PyTorch on the host, float64, rounded once to float32), not the code being measured: the observations depend on the seeds,
+    numpy and torch only, so every build benchmarked with the same arguments receives the same bytes (inputs_sha256 in the
+    result line), and a build whose forward pass is wrong leaves residuals that show in its loss and gradients."""
+    from tests import util_stage3 as U
+    cfg = CONFIGS[config]
+    of = cfg['optim_floor']
+    B, T = prob['obs']['joints2d'].shape[:2]
+    port = U.build_port(B, T, getattr(synth, cfg['weights']), of, prob, dtype=torch.float64)
+    params = {k: torch.as_tensor(prob['params'][k], dtype=torch.float64) for k in U.PARAM_NAMES + (['floor_plane'] if of else [])}
+    obs = {k: U.obs_to(prob['obs'][k], 'cpu') for k in U.obs_keys(of)}
     with torch.no_grad():
-        _, _, _, _, cam_pred = mo.stage3_forward(obs)
+        _, _, inter = port.closure(params, obs)
+    cam = inter['cam_pred']
     if config == 'amass':
-        v = cam_pred['verts3d'].cpu().numpy()
+        v = cam['verts3d'].numpy()
         rng = np.random.RandomState(5)
         occl = np.isinf(prob['obs']['verts3d'])
         prob['obs']['verts3d'] = np.where(occl, np.inf, v + rng.randn(*v.shape) * 0.01).astype(np.float32)
         return prob
-    from humor_b200.fitting_loss import SMPL2OP
-    j = cam_pred['Jtr'][:, :, SMPL2OP].cpu().numpy()
-    rng = np.random.RandomState(5)
-    f, c = np.asarray(synth.CAM_F), np.asarray(synth.CAM_C)
-    prob['obs']['joints2d'][..., :2] = (j[..., :2] / j[..., 2:3] * f + c + rng.randn(*j.shape[:3], 2) * 2.0).astype(np.float32)
-    return prob
+    return U.project_joints2d(prob, torch.cat([cam['joints3d'], cam['joints3d_extra']], 2).numpy(), seed=5, noise=2.0)
+
+
+def inputs_sha256(prob, obs_keys):
+    """SHA-256 of every array the timed step reads (variables and observations, in a fixed order)."""
+    h = hashlib.sha256()
+    for part in (prob['params'], prob['obs']):
+        keys = sorted(part) if part is prob['params'] else obs_keys
+        for k in keys:
+            a = np.ascontiguousarray(part[k])
+            h.update(f'{k} {a.dtype.str} {a.shape}'.encode() + a.tobytes())
+    return h.hexdigest()
 
 
 def run_product(args):
@@ -155,11 +173,11 @@ def run_product(args):
     _ext.check(_ext.lib().humor_lbs_configure(args.lbs_skin, args.lbs_blend, args.lbs_slab), 'humor_lbs_configure')
     B, T = args.batch, args.seq_len
     OBS_KEYS = CONFIGS[args.config]['obs']
-    prob = build_problem(B, T, seed=4 + rank, config=args.config)
+    prob = project_obs(build_problem(B, T, seed=4 + rank, config=args.config), args.config)
     mo = make_optimizer(B, T, prob, dev, args.config)
-    prob = project_obs_from_product(mo, prob, dev, args.config)
     # global frame intervals of this rank's block of sub-sequences (one video split across the ranks)
     prob['obs']['seq_interval'] = prob['obs']['seq_interval'] + rank * B * (T - 10)
+    inputs_digest = inputs_sha256(prob, OBS_KEYS)
     if world > 1 and 'seq_interval' in OBS_KEYS and not args.no_halo:
         from humor_b200.parallel import Shard
         mo.shard = Shard.from_env(ov_max=16)
@@ -199,6 +217,8 @@ def run_product(args):
         marks[i + 1].record()
     e1.record()
     barrier()
+    # what the last timed step returned, copied on the device; written to disk once the clock sampling has ended
+    last = (loss.detach().clone(), {n: getattr(mo, n).grad.detach().clone() for n in names}) if args.dump_outputs and rank == 0 else None
     ms = e0.elapsed_time(e1)
     per = torch.tensor([marks[i].elapsed_time(marks[i + 1]) for i in range(args.steps)], device=dev)
     per_all = per[None]
@@ -225,6 +245,9 @@ def run_product(args):
     clocks = sampler.stop(row0, timed_rows) if rank == 0 else None
     if clocks is not None:
         clocks['untimed_steps_under_sampling'] = extra
+    if last is not None:
+        dump_outputs(args.dump_outputs, *last)
+        last = None
     # ---- end-to-end timing: host params/observations in pinned memory in, loss + gradients out, every step
     host_in = {n: torch.as_tensor(prob['params'][n]).pin_memory() for n in names}
     host_obs = {k: torch.as_tensor(prob['obs'][k]).pin_memory() for k in OBS_KEYS}
@@ -292,7 +315,7 @@ def run_product(args):
                 'ms_per_step': ms_e2e / args.steps},
         'gpu_launches': int(launches), 'gpu_launches_per_step': launches / args.steps, 'per_step_ms': per_step,
         'clocks': clocks, 'roofline': roof, 'step_breakdown_ms': shares, 'cpu_baseline': cpu,
-        'torch_cuda_port': torch_cuda, 'result_check': result_check,
+        'torch_cuda_port': torch_cuda, 'result_check': result_check, 'inputs_sha256': inputs_digest,
         'lbs_bytes_roofline_frac_of_step': value * (2.0 + 3.0 / T) * (LBS_BYTES_FWD + LBS_BYTES_BWD) / (hbm_peak * 1e9),
     }
     # The two context numbers run in bounded child processes AFTER the measurement, inside what is left of the run's time
@@ -322,6 +345,26 @@ def run_product(args):
         out['step_candidates'] = step_candidates(args, result_check)
     _PARTIAL = None
     print(json.dumps(out))
+
+
+def dump_outputs(path, loss, grads):
+    """What the last timed step returned to its caller: loss.npy (1,) and grad_<variable>.npy for every stage-3 variable, all
+    float32 (2 961 floats per sub-sequence in the RGB config: 3.0 MB at B = 256).  Every variable leads with the sub-sequence
+    axis; when the files would exceed DUMP_LIMIT_BYTES, the same seeded sample of sub-sequences is kept of each and
+    sample_rows.npy (float64) lists it, the sample sized so that all files, headers included, stay within the limit."""
+    os.makedirs(path, exist_ok=True)
+    out = {'grad_' + n: g.detach().float().cpu().numpy() for n, g in grads.items()}
+    B = next(iter(out.values())).shape[0]
+    row_bytes = sum(a.nbytes for a in out.values()) // B
+    headers = NPY_HEADER_BYTES * (len(out) + 2)                  # the gradients, loss.npy and sample_rows.npy
+    if B * row_bytes + 4 + headers > DUMP_LIMIT_BYTES:
+        keep = (DUMP_LIMIT_BYTES - 4 - headers) // (row_bytes + 8)
+        rows = np.sort(np.random.RandomState(0).choice(B, keep, replace=False))
+        out = {k: a[rows] for k, a in out.items()}
+        out['sample_rows'] = rows.astype(np.float64)
+    out['loss'] = loss.detach().float().reshape(1).cpu().numpy()
+    for k, a in out.items():
+        np.save(os.path.join(path, k + '.npy'), a)
 
 
 def lbs_roofline(mo, B, T, dev, hbm_peak, peak_kind):
@@ -657,9 +700,17 @@ def main():
     ap.add_argument('--no-halo', action='store_true', help='diagnostic: N independent replicas (no overlap coupling between ranks, no collective)')
     ap.add_argument('--no-graph', action='store_true', help='evaluate the closure eagerly instead of replaying a CUDA graph')
     ap.add_argument('--port-cuda', default='', help='comma list of batch sizes: time the oracle port as eager PyTorch on cuda:0')
+    ap.add_argument('--dump-outputs', default='', metavar='DIR',
+                    help='after the timed steps, write the loss and gradients the last of them returned as DIR/<name>.npy '
+                         '(float32, at most 64 MB; with several GPUs, those of rank 0). The inputs do not depend on the '
+                         'build, so dumps of two builds run with the same arguments can be compared output for output')
     ap.add_argument('--_cpu-child', dest='cpu_child', action='store_true', help=argparse.SUPPRESS)
     ap.add_argument('--cpu-threads', type=int, default=0, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'humor_b200' or args.port_cuda):
+        ap.error('--dump-outputs writes what the timed humor_b200 step returned: not with --impl reference or --port-cuda')
     if args.cpu_child:
         import warnings
         warnings.filterwarnings('ignore')

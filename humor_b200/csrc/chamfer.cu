@@ -3,7 +3,7 @@
 // (pybind surface chamfer_distance.cpp:180-185; used by FittingLoss.points3d_loss, fitting_loss.py:378-396).
 //
 // Semantics follow the reference's CPU path `nnsearch` (chamfer_distance.cpp:58-87) exactly, so results are
-// bit-identical to it (tests compare against the compiled reference, oracle/_ref/cd_ref.so):
+// bit-identical to it (tests compare against what the compiled reference wrote, tests/golden/*chamfer_*.npz):
 //   d(j,k) = ((dx*dx) + (dy*dy)) + (dz*dz)   with dx = target - query, every operation rounded separately
 //            (explicit __fmul_rn/__fadd_rn: nvcc must not contract them into FMAs),
 //   the first target attaining the strict minimum wins (`k == 0 || d < best`), a NaN distance never replaces

@@ -14,11 +14,13 @@ Contents
                   reference file:line it follows.  Portable: travels to the GPU box.
   ref_import.py   imports the UNMODIFIED reference from /root/reference (this container only)
                   behind a ``smplx`` stub backed by smplh_lbs.py.
-  make_golden.py  runs the real reference here and writes tests/golden/*.npz.
+  make_golden.py  runs the real reference and writes tests/golden/stage*.npz.
+  make_golden_ref.py  runs the real reference on the inputs of the other comparison tests and
+                  writes tests/golden/ref_*.npz.
 
 Parity pinning: the reference ships no tests or golden vectors (SURVEY.md §4).  The port is
-pinned against the reference *executed here* (tests/test_oracle_vs_reference.py, skipped when
-/root/reference is absent) and against the committed fixtures generated by make_golden.py.
+pinned against the committed fixtures the make_golden*.py scripts generated from the
+reference; no test needs the reference itself, so every comparison runs on every machine.
 The LBS restatement has no runnable third-party source to check against (smplx is not
 installable offline): **LBS parity is pinned only by the analytic known-answer cases** in
 tests/test_oracle_lbs.py (zero pose, rigid root rotation, hand-column independence).

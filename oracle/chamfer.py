@@ -9,9 +9,9 @@ Follows (paths relative to /root/reference/humor):
   robust_std / bisquare_robust_weights / apply_robust_weighting   fitting/fitting_utils.py:192-248
   points3d_loss    fitting/fitting_loss.py:378-396
 
-Pinned: bit-exact against the reference's own C++ compiled from its sources in place (oracle/build_ref.py ->
-oracle/_ref/cd_ref.so; tests/test_oracle_chamfer.py) and against tests/golden/chamfer_*.npz, which that compiled
-reference wrote (oracle/make_golden_chamfer.py).  fp32 arithmetic in the reference's order: ((dx*dx)+(dy*dy))+(dz*dz)
+Pinned: bit-exact against what the reference's own C++, compiled from its sources in place (oracle/build_ref.py ->
+oracle/_ref/cd_ref.so), wrote: tests/golden/chamfer_*.npz (oracle/make_golden_chamfer.py) and
+tests/golden/ref_chamfer_*.npz (oracle/make_golden_ref.py); tests/test_oracle_chamfer.py.  fp32 arithmetic in the reference's order: ((dx*dx)+(dy*dy))+(dz*dz)
 with dx = target - query, first strict minimum wins.
 """
 import numpy as np

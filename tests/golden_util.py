@@ -1,8 +1,24 @@
+import hashlib
 import os
 import numpy as np
 from humor_b200 import synth
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
+
+
+def npz_digests(root, names=None):
+    """{'<dir relative to root>:<file>:<key>': 'dtype shape sha256'} of every array in the npz files under `root` (or of the
+    files `names` in `root`): two trees have equal digests exactly when they hold the same files, keys, dtypes and bytes."""
+    out = {}
+    for d, _, files in os.walk(root):
+        for fn in sorted(files):
+            if fn.endswith('.npz') and (names is None or (d == root and fn in names)):
+                z = np.load(os.path.join(d, fn))
+                for k in z.files:
+                    a = np.ascontiguousarray(z[k])
+                    key = ':'.join(([] if names is not None else [os.path.relpath(d, root)]) + [fn, k])
+                    out[key] = '%s %s %s' % (a.dtype.str, a.shape, hashlib.sha256(a.tobytes()).hexdigest())
+    return out
 CASES = ['stage3_rgb', 'stage3_rgb_phase1', 'stage3_rgb_refine', 'stage3_amass', 'stage3_proxd', 'stage3_rgb_xbatch']
 
 

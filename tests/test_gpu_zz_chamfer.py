@@ -1,7 +1,7 @@
 """GPU parity of the chamfer nearest-neighbour kernels (csrc/chamfer.cu through the C-ABI) and of the points3d
 energy built on them.  Bit-exact against (1) the golden vectors written by the reference's own compiled C++
-(tests/golden/chamfer_*.npz), (2) the CPU oracle port on ragged sizes, (3) the compiled reference itself when
-oracle/_ref/cd_ref.so travelled to the box; closure-level parity against the PROX-RGBD golden case of the
+(tests/golden/chamfer_*.npz), (2) the CPU oracle port on ragged sizes, (3) the compiled reference's forward on larger
+random clouds (tests/golden/ref_chamfer_gpu.npz); closure-level parity against the PROX-RGBD golden case of the
 unmodified reference (stage3_proxd) and the oracle port; size-independent properties at the full PROX size
 (4096 observed points against 6890 vertices).
 
@@ -70,19 +70,15 @@ def test_kernels_match_port_on_ragged_sizes(b, n, m):
 
 
 def test_matches_compiled_reference_when_present():
-    from oracle.build_ref import load_cd_ref
+    """Bit-exact against the compiled reference module's forward on 4 x 600 against 4 x 1500 random points, stored by
+    oracle/make_golden_ref.py; always runs (the name dates from when the module itself had to be present)."""
     from humor_b200.chamfer import chamfer_nn
-    cd = load_cd_ref()
-    if cd is None:
-        pytest.skip('oracle/_ref/cd_ref.so did not travel to this box')
-    rng = np.random.default_rng(11)
-    a = rng.normal(size=(4, 600, 3)).astype(np.float32)
-    c = rng.normal(size=(4, 1500, 3)).astype(np.float32)
-    d1, d2 = torch.zeros(4, 600), torch.zeros(4, 1500)
-    i1, i2 = torch.zeros(4, 600, dtype=torch.int), torch.zeros(4, 1500, dtype=torch.int)
-    cd.forward(torch.from_numpy(a), torch.from_numpy(c), d1, d2, i1, i2)
+    from tests import ref_inputs as R
+    ref = R.fixture('ref_chamfer_gpu')
+    a, c = R.chamfer_gpu_case()
     e1, e2, j1, j2 = chamfer_nn(dev(a), dev(c))
-    assert torch.equal(e1.cpu(), d1) and torch.equal(e2.cpu(), d2) and torch.equal(j1.cpu(), i1) and torch.equal(j2.cpu(), i2)
+    assert np.array_equal(bits(e1.cpu().numpy()), bits(ref['dist1'])) and np.array_equal(bits(e2.cpu().numpy()), bits(ref['dist2']))
+    assert np.array_equal(j1.cpu().numpy(), ref['idx1']) and np.array_equal(j2.cpu().numpy(), ref['idx2'])
 
 
 def test_full_size_properties():

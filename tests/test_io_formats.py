@@ -1,38 +1,16 @@
-"""On-disk formats (humor_b200/io_formats.py) against the reference's own readers/writers executed live in the build
-container (skipped where /root/reference is absent) and against known answers that hold everywhere.  CPU only."""
-import json
+"""On-disk formats (humor_b200/io_formats.py) against what the reference's own readers/writers produced on the same
+inputs (tests/golden/ref_io_formats.npz, written by oracle/make_golden_ref.py from the inputs of tests/ref_inputs.py) and
+against known answers.  CPU only."""
 import os
-import sys
-import types
 
 import numpy as np
 import pytest
 import torch
 
 from humor_b200 import io_formats as F
-from oracle import ref_import
-
-needs_ref = pytest.mark.skipif(not ref_import.available(), reason='/root/reference is only present in the build container')
-
-
-def write_openpose_dir(path, T, seed=0, empty=(3,)):
-    rng = np.random.RandomState(seed)
-    os.makedirs(path, exist_ok=True)
-    frames = []
-    for t in range(T):
-        kp = np.concatenate([rng.rand(25, 2) * 1000, rng.rand(25, 1)], 1)
-        people = [] if t in empty else [{'pose_keypoints_2d': kp.reshape(-1).tolist()},
-                                        {'pose_keypoints_2d': (kp * 0.5).reshape(-1).tolist()}]    # 2nd person ignored
-        with open(os.path.join(path, 'frame_%06d_keypoints.json' % t), 'w') as f:
-            json.dump({'version': 1.3, 'people': people}, f)
-        frames.append(np.zeros((25, 3)) if t in empty else kp)
-    return np.stack(frames, 0)
-
-
-def ref_mods():
-    ref = ref_import.load()
-    np.float = float                     # the reference predates numpy 1.24 (fitting_utils.py:30,33-34)
-    return ref
+from tests import ref_inputs as R
+from tests.golden_util import npz_digests
+from tests.ref_inputs import write_openpose_dir
 
 
 def test_read_keypoints_known_answer(tmp_path):
@@ -43,33 +21,21 @@ def test_read_keypoints_known_answer(tmp_path):
         assert np.array_equal(got, kp[t])
 
 
-@needs_ref
 def test_read_keypoints_matches_reference(tmp_path):
-    ref = ref_mods()
-    write_openpose_dir(str(tmp_path), 6)
-    for p in F.keypoint_paths(str(tmp_path)):
-        assert np.array_equal(F.read_keypoints(p), ref.fitting_utils.read_keypoints(p))
+    """fitting_utils.read_keypoints's arrays for the same OpenPose files (one frame without a person)."""
+    want = R.fixture('ref_io_formats')['read_keypoints']
+    write_openpose_dir(str(tmp_path), R.KEYPOINT_FRAMES)
+    got = np.stack([F.read_keypoints(p) for p in F.keypoint_paths(str(tmp_path))])
+    assert got.dtype == want.dtype and np.array_equal(got, want)
 
 
-def reference_intervals(num_frames, seq_len, overlap_len):
-    """rgb_dataset.py:74-99 executed literally (the module itself needs cv2, which this image lacks)."""
-    import math
-    src = open('/root/reference/humor/datasets/rgb_dataset.py').read().splitlines()
-    a = next(i for i, l in enumerate(src) if l.strip() == 'seq_intervals = []')
-    b = next(i for i, l in enumerate(src) if l.strip() == 'seq_intervals = [(0, self.seq_len)]')
-    body = '\n'.join(l[8:] for l in src[a:b + 1])          # rgb_dataset.py:74-99
-    ns = types.SimpleNamespace(seq_len=seq_len, overlap_len=overlap_len)
-    env = {'self': ns, 'num_frames': num_frames, 'math': math, 'print': lambda *a, **k: None}
-    exec(body, env)
-    return [tuple(x) for x in env['seq_intervals']], ns.overlap_len
-
-
-@needs_ref
-@pytest.mark.parametrize('F_,L,o', [(300, 60, 10), (301, 60, 10), (125, 60, 10), (1000, 60, 10), (77, 30, 5), (61, 60, 10)])
+@pytest.mark.parametrize('F_,L,o', R.SPLITS)
 def test_split_intervals_matches_reference(F_, L, o):
+    """The windows and overlap of the reference's RGB-video split (rgb_dataset.py:74-99)."""
+    ref = R.fixture('ref_io_formats')
     got, ov = F.split_intervals(F_, L, o)
-    want, ov_ref = reference_intervals(F_, L, o)
-    assert got == want and ov == ov_ref
+    want = [tuple(int(x) for x in r) for r in ref['split:%d:%d:%d' % (F_, L, o)]]
+    assert got == want and ov == int(ref['split_overlap:%d:%d:%d' % (F_, L, o)])
 
 
 def test_split_intervals_properties():
@@ -93,81 +59,42 @@ def test_load_rgb_video(tmp_path):
     assert gt['name'][1] == 'rgb_video_0001'
 
 
-def fake_results(B, T, rng):
-    t = lambda *s: torch.tensor(rng.randn(*s).astype(np.float32))
-    optim = {'betas': t(B, 16), 'trans': t(B, T, 3), 'root_orient': t(B, T, 3), 'pose_body': t(B, T, 63),
-             'latent_pose': t(B, T, 32), 'latent_motion': t(B, T - 1, 48), 'contacts': (t(B, T, 22) > 0).float(),
-             'floor_plane': t(B, 4)}
-    stages = {'stage3': {'prior_trans': t(B, T, 3), 'prior_root_orient': t(B, T, 3)}}
-    obs = {'joints2d': t(B, T, 25, 3), 'floor_plane': t(B, 4), 'seq_interval': torch.tensor([[i * (T - 3), i * (T - 3) + T] for i in range(B)], dtype=torch.int)}
-    gt = {'cam_matx': t(B, 3, 3), 'name': ['v_%04d' % i for i in range(B)]}
-    return optim, stages, obs, gt
-
-
-def npz_equal(a, b):
-    A, B_ = np.load(a, allow_pickle=True), np.load(b, allow_pickle=True)
-    assert sorted(A.files) == sorted(B_.files), (a, A.files, B_.files)
-    for k in A.files:
-        assert A[k].dtype == B_[k].dtype and np.array_equal(A[k], B_[k]), (a, k)
-
-
-@needs_ref
-@pytest.mark.parametrize('data_type,with_smpl_gt', [('RGB', False), ('AMASS', True), ('PROX-RGBD', True)])
+@pytest.mark.parametrize('data_type,with_smpl_gt', R.SAVE_CASES)
 def test_save_optim_result_matches_reference(tmp_path, data_type, with_smpl_gt):
-    ref = ref_mods()
-    rng = np.random.RandomState(0)
-    B, T = 3, 7
-    optim, stages, obs, gt = fake_results(B, T, rng)
-    if with_smpl_gt:
-        g = lambda *s: torch.tensor(rng.randn(*s).astype(np.float32))
-        gt.update(betas=g(B, 16) if data_type.startswith('PROX') else g(B, T, 16), trans=g(B, T, 3), root_orient=g(B, T, 3),
-                  pose_body=g(B, T, 63), contacts=g(B, T, 22))
-    img = [tuple('f%d_b%d.png' % (t, b) for b in range(B)) for t in range(T)]
-    dirs = {}
-    for who in ('ref', 'new'):
-        dirs[who] = [str(tmp_path / who / ('s%d' % b)) for b in range(B)]
-        for d in dirs[who]:
-            os.makedirs(d)
-    ref.fitting_utils.save_optim_result(dirs['ref'], optim, stages, gt, obs, data_type, optim_floor=True, obs_img_paths=img)
-    F.save_optim_result(dirs['new'], optim, stages, gt, obs, data_type, optim_floor=True, obs_img_paths=img)
-    for a, b in zip(dirs['ref'], dirs['new']):
-        assert sorted(os.listdir(a)) == sorted(os.listdir(b))
-        for fn in os.listdir(a):
-            npz_equal(os.path.join(a, fn), os.path.join(b, fn))
+    """Every file fitting_utils.save_optim_result writes for these inputs: same files, keys, dtypes and bytes."""
+    optim, stages, gt, obs, img, B = R.save_case(data_type, with_smpl_gt)
+    dirs = [str(tmp_path / ('s%d' % b)) for b in range(B)]
+    for d in dirs:
+        os.makedirs(d)
+    F.save_optim_result(dirs, optim, stages, gt, obs, data_type, optim_floor=True, obs_img_paths=img)
+    want = R.ref_digests('save:%s:' % data_type)
+    got = npz_digests(str(tmp_path))
+    assert sorted(got) == sorted(want)
+    for k in want:
+        assert got[k] == want[k], k
 
 
-@needs_ref
 def test_stitched_result_matches_reference(tmp_path):
-    """final_results/ against the reference's save_rgb_stitched_result run with its own BodyModel (restated smplx behind
-    it) for the prior-frame copy; the files that do not depend on SMPL must be identical."""
-    ref = ref_mods()
-    sys.modules.setdefault('cv2', types.ModuleType('cv2'))       # imported, never used, by the reference function
+    """final_results/ against what the reference's save_rgb_stitched_result wrote from the same per-sequence files (run with
+    its own BodyModel, restated smplx behind it, for the prior-frame copy); the files that do not depend on SMPL must be
+    identical."""
     from oracle.ref_closure import asset_npz
-    rng = np.random.RandomState(1)
-    B, T = 3, 8
-    optim, stages, obs, gt = fake_results(B, T, rng)
-    optim['floor_plane'] = torch.tensor([[0.0, -1.0, 0.05, -0.6]] * B)
-    optim['trans'][..., 2] += 3.0
-    img = [tuple('f%d_b%d.png' % (t, b) for b in range(B)) for t in range(T)]
-    roots = {}
-    for who in ('ref', 'new'):
-        roots[who] = str(tmp_path / who)
-        dirs = [os.path.join(roots[who], 's%d' % b) for b in range(B)]
-        for d in dirs:
-            os.makedirs(d)
-        F.save_optim_result(dirs, optim, stages, gt, obs, 'RGB', obs_img_paths=img)
-        F.write_meta(dirs, asset_npz())
-        roots[who + '_dirs'] = dirs
+    optim, stages, gt, obs, img, B = R.stitched_case()
+    dirs = [str(tmp_path / ('s%d' % b)) for b in range(B)]
+    for d in dirs:
+        os.makedirs(d)
+    F.save_optim_result(dirs, optim, stages, gt, obs, 'RGB', obs_img_paths=img)
+    F.write_meta(dirs, asset_npz())
     iv = [tuple(int(x) for x in r) for r in obs['seq_interval']]
-    import contextlib
-    import io
-    with contextlib.redirect_stdout(io.StringIO()):
-        ref.fitting_utils.save_rgb_stitched_result(iv, roots['ref_dirs'], roots['ref'], torch.device('cpu'), asset_npz(), 16, True)
-    F.save_rgb_stitched_result(iv, roots['new_dirs'], roots['new'])
-    for fn in ('gt_results.npz', 'observations.npz', 'stage3_results.npz'):
-        npz_equal(os.path.join(roots['ref'], 'final_results', fn), os.path.join(roots['new'], 'final_results', fn))
-    assert open(os.path.join(roots['ref'], 'final_results', 'meta.txt')).read() == open(os.path.join(roots['new'], 'final_results', 'meta.txt')).read()
-    st = F.stitch_subsequences(iv, roots['new_dirs'])
+    F.save_rgb_stitched_result(iv, dirs, str(tmp_path))
+    final = str(tmp_path / 'final_results')
+    want = R.ref_digests('stitched:')
+    got = npz_digests(final, R.STITCHED_FILES)
+    assert sorted(got) == sorted(want)
+    for k in want:
+        assert got[k] == want[k], k
+    assert open(os.path.join(final, 'meta.txt')).read() == R.fixture('ref_io_formats')['stitched_meta'].item().replace('<asset>', asset_npz())
+    st = F.stitch_subsequences(iv, dirs)
     assert st['trans'].shape[0] == iv[-1][1] and st['joints2d'].shape[0] == iv[-1][1] and len(st['img_paths']) == iv[-1][1]
 
 

@@ -1,12 +1,12 @@
 """CPU tests that pin the oracle: (1) the torch port against the committed fixtures produced by the REAL reference
-(oracle/make_golden.py); (2) against the reference executed live when /root/reference exists; (3) analytic
-known answers for the restated smplx LBS (no runnable third-party source exists: LBS parity is pinned only here)."""
+(oracle/make_golden.py, oracle/make_golden_ref.py); (2) analytic known answers for the restated smplx LBS (no runnable
+third-party source exists: LBS parity is pinned only here)."""
 import numpy as np
 import pytest
 import torch
 
 from humor_b200 import synth
-from oracle import ref_import
+from tests import ref_inputs as R
 from tests import util_stage3 as U
 from tests.golden_util import CASES, load_case, check_against_golden
 
@@ -39,38 +39,31 @@ def test_port_stage12_matches_reference_golden(name):
     assert np.abs(inter['pred']['verts3d'].detach().numpy() - g['pred_verts3d']).max() < 1e-5
 
 
-@pytest.mark.skipif(not ref_import.available(), reason='/root/reference is only present in the build container')
-@pytest.mark.parametrize('optim_floor,nsteps,scale', [(True, None, 1.0), (True, 5, 1.0), (False, None, 2.4)])
+@pytest.mark.parametrize('optim_floor,nsteps,scale', R.STAGE3_SEED31)
 def test_port_matches_live_reference(optim_floor, nsteps, scale):
-    from oracle import ref_closure
-    B, T = 4, 9          # not 3: see oracle/make_golden.py (torch.cross default-dim quirk of the reference)
-    W = synth.RGB_STAGE3_WEIGHTS if optim_floor else synth.AMASS_STAGE3_WEIGHTS
-    prob = synth.make_stage3_problem(B, T, seed=31, overlap=3, cam=optim_floor)
-    ref, mo, _, _ = ref_closure.build(B, T, W, optim_floor, prob['cam_mat'] if optim_floor else None)
-    names = ref_closure.set_params(mo, prob['params'])
-    obs = {k: torch.as_tensor(prob['obs'][k]) for k in U.obs_keys(optim_floor)}
-    loss, stats, _ = ref_closure.stage3_closure(ref, mo, {k: v.clone() for k, v in obs.items()}, nsteps, scale)
+    """Loss, every energy term and every gradient of the port against the reference's Stage-III closure on the seeded
+    synthetic problem as generated (observations included), stored by oracle/make_golden_ref.py (the name dates from when
+    the reference was executed inside the test)."""
+    g = R.fixture(R.stage3_name(optim_floor, nsteps, scale))
+    B, T, W, prob = R.stage3_case(optim_floor)
     port = U.build_port(B, T, W, optim_floor, prob)
     l2, g2, aux = U.closure_port(port, prob, optim_floor, nsteps, scale)
-    assert abs(l2 - loss.item()) <= 2e-6 * max(1.0, abs(loss.item()))
-    for k, v in stats.items():
-        assert abs(aux['stats'][k] - float(v)) <= 2e-5 * max(1.0, abs(float(v))), k
-    for n in names:
-        ref_g = getattr(mo, n).grad
-        assert float((g2[n] - ref_g).abs().max() / (ref_g.abs().max() + 1e-8)) < 1e-4, n
+    assert sorted(k[5:] for k in g if k.startswith('grad_')) == sorted(g2)
+    check_against_golden(g, l2, aux['stats'], g2, loss_tol=2e-6, stat_tol=2e-5, grad_tol=1e-4)
 
 
 def test_reference_rotation_helpers_match_port():
-    if not ref_import.available():
-        pytest.skip('/root/reference absent')
+    """Port rotation helpers against the reference's batch_rodrigues / rotation_matrix_to_angle_axis /
+    compute_world2aligned_mat on 500 seeded axis-angle vectors (stored by oracle/make_golden_ref.py)."""
     from oracle.stage3_port import mat2aa, world2aligned
     from oracle.smplh_lbs import rodrigues
-    ref = ref_import.load()
-    aa = torch.randn(500, 3) * 1.3
-    R = rodrigues(aa)
-    assert torch.allclose(R, ref.transforms.batch_rodrigues(aa), atol=1e-6)
-    assert torch.allclose(mat2aa(R), ref.transforms.rotation_matrix_to_angle_axis(R), atol=1e-6)
-    assert torch.allclose(world2aligned(R), ref.transforms.compute_world2aligned_mat(R), atol=1e-6)
+    g = R.fixture('ref_rotations')
+    aa = R.rotation_inputs()
+    assert torch.equal(aa, torch.from_numpy(g['aa']))         # the fixture was made from these inputs
+    rot = torch.from_numpy(g['rodrigues'])
+    assert torch.allclose(rodrigues(aa), rot, atol=1e-6)
+    assert torch.allclose(mat2aa(rot), torch.from_numpy(g['mat2aa']), atol=1e-6)
+    assert torch.allclose(world2aligned(rot), torch.from_numpy(g['world2aligned']), atol=1e-6)
 
 
 # ------------------------------------------------------------------------------------------------ LBS known answers

@@ -1,6 +1,6 @@
 """Pins the chamfer oracle (oracle/chamfer.py): bit-exact against the golden vectors the COMPILED reference wrote
-(tests/golden/chamfer_*.npz, oracle/make_golden_chamfer.py) and, when oracle/_ref/cd_ref.so is present, against the
-reference module itself on fresh random inputs.  CPU only."""
+(tests/golden/chamfer_*.npz, oracle/make_golden_chamfer.py; tests/golden/ref_chamfer_random.npz,
+oracle/make_golden_ref.py on the inputs of tests/ref_inputs.py).  CPU only."""
 import glob
 import os
 
@@ -9,7 +9,7 @@ import pytest
 import torch
 
 from oracle import chamfer as oc
-from oracle.build_ref import load_cd_ref
+from tests import ref_inputs as R
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = sorted(glob.glob(os.path.join(ROOT, 'tests', 'golden', 'chamfer_*.npz')))
@@ -44,25 +44,16 @@ def test_ties_take_first_minimum():
 
 
 def test_port_matches_live_reference():
-    cd = load_cd_ref()
-    if cd is None:
-        pytest.skip('oracle/_ref/cd_ref.so not built (python oracle/build_ref.py)')
-    rng = np.random.default_rng(7)
-    for b, n, m in [(1, 1, 1), (2, 5, 3), (3, 129, 1025), (1, 700, 2)]:
-        a = rng.normal(size=(b, n, 3)).astype(np.float32)
-        c = rng.normal(size=(b, m, 3)).astype(np.float32)
-        d1, d2 = torch.zeros(b, n), torch.zeros(b, m)
-        i1, i2 = torch.zeros(b, n, dtype=torch.int), torch.zeros(b, m, dtype=torch.int)
-        cd.forward(torch.from_numpy(a), torch.from_numpy(c), d1, d2, i1, i2)
+    """Bit-exact against the compiled reference module's forward / backward on random clouds of several shapes, stored by
+    oracle/make_golden_ref.py (the name dates from when the module was called inside the test)."""
+    ref = R.fixture('ref_chamfer_random')
+    for b, n, m, a, c, gd1, gd2 in R.chamfer_random_cases():
+        r = {k.split(':')[1]: v for k, v in ref.items() if k.startswith('%d_%d_%d:' % (b, n, m))}
         p1, p2, q1, q2 = oc.chamfer_forward(a, c)
-        assert np.array_equal(q1, i1.numpy()) and np.array_equal(q2, i2.numpy())
-        assert np.array_equal(p1, d1.numpy()) and np.array_equal(p2, d2.numpy())
-        gd1 = rng.normal(size=(b, n)).astype(np.float32)
-        gd2 = rng.normal(size=(b, m)).astype(np.float32)
-        g1, g2 = torch.zeros(b, n, 3), torch.zeros(b, m, 3)
-        cd.backward(torch.from_numpy(a), torch.from_numpy(c), g1, g2, torch.from_numpy(gd1), torch.from_numpy(gd2), i1, i2)
+        assert np.array_equal(q1, r['idx1']) and np.array_equal(q2, r['idx2'])
+        assert np.array_equal(p1, r['dist1']) and np.array_equal(p2, r['dist2'])
         o1, o2 = oc.chamfer_backward(a, c, gd1, gd2, q1, q2)
-        assert np.array_equal(o1, g1.numpy()) and np.array_equal(o2, g2.numpy())
+        assert np.array_equal(o1, r['grad_xyz1']) and np.array_equal(o2, r['grad_xyz2'])
 
 
 def test_empty_target_cloud():
